@@ -16,6 +16,8 @@ src/coverage.h:412-441). configs[1] names ~5 M split/discordant reads -> 10 M re
 
 Launch: python bench.py [--gpus N --steps K --warmup W] ; N>1 under torchrun (one rank per GPU).
         python bench.py --impl reference ...   times the reference CPU path on the same config.
+        python bench.py --dump-outputs DIR ...  also writes what the last timed step computed to DIR (see dump_outputs;
+                                                bench_outputs/ is git-ignored for this).
 """
 import argparse
 import json
@@ -49,6 +51,27 @@ def make_batch(n_jobs, seed):
         parts.append(b)
     assert base < 2 ** 32
     return {k: np.concatenate([p[k] for p in parts]) for k in parts[0]}
+
+
+DUMP_BUDGET = 64 << 20
+DUMP_SEED = 20240917
+
+
+def dump_outputs(out_dir, dist, world, rank):
+    """Writes the edit distances of the last timed step (what a caller of dgpu_edit_distance_dev receives, one int32 per job, -1 where the
+    bound k was exceeded) as float32 to out_dir/edit_distance.npy (N > 1: edit_distance_rank<r>.npy per rank). The inputs are seeded, so two
+    builds given the same arguments can be compared output for output. Above the 64 MB budget (shared by all ranks) a fixed, seeded sample
+    of job indices is written instead, in job order, with the indices in edit_distance_index.npy (float64, exact)."""
+    os.makedirs(out_dir, exist_ok=True)
+    sfx = "" if world == 1 else f"_rank{rank}"
+    n = len(dist)
+    cap = DUMP_BUDGET // world // 4
+    if n > cap:
+        # indices (8 bytes each as float64) and values (4 bytes) share the budget
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=DUMP_BUDGET // world // 12, replace=False))
+        np.save(os.path.join(out_dir, f"edit_distance_index{sfx}.npy"), idx.astype(np.float64))
+        dist = dist[idx]
+    np.save(os.path.join(out_dir, f"edit_distance{sfx}.npy"), dist.astype(np.float32))
 
 
 def algorithmic_counts(b):
@@ -587,7 +610,11 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-families", action="store_true")
     ap.add_argument("--no-pipeline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the edit distances of the last timed step to DIR/*.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
 
@@ -683,6 +710,8 @@ def main():
     ev1.record()
     barrier()
     total_ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, d_dist.cpu().numpy(), world, rank)     # before the untimed runs below reuse d_dist
     launches = ctx.launches - l0
     # dominant-kernel span (library-side CUDA events on the launching stream), measured outside the loop timing
     kms = []

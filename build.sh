@@ -25,18 +25,19 @@ g++ -std=c++17 -O2 -fPIC -shared -Wall -Wno-sign-compare -o delly_b200/libdelly_
   -Ldelly_b200 -l:libdelly_b200.so -Wl,-rpath,'$ORIGIN'
 echo "built delly_b200/libdelly_b200_host.so"
 # the drop-in binding `delly_b200 sr|lr` (bindings/): htslib IO around the batched host mirrors. htslib = the reference's vendored submodule,
-# compiled by tools/build_htslib.sh where the reference tree exists (here); on the GPU box the prebuilt archive and binary are used.
+# compiled with its public headers into oracle/_ref/hts by tools/build_htslib.sh where the reference tree exists; elsewhere the archive and
+# headers already under oracle/_ref/hts (built with the checkers) are used, as are the MEI templates extracted next to them.
 bash tools/build_htslib.sh
 python tools/extract_mei.py > /dev/null
-HTSINC=${REF:-/root/reference}/src/htslib
-if [ -d "$HTSINC" ] && [ -f third_party/_hts/libhts.a ]; then
+HTS=oracle/_ref/hts
+if [ -f $HTS/include/htslib/sam.h ] && [ -f $HTS/libhts.a ]; then
   mkdir -p delly_b200/bin
-  g++ -std=c++17 -O2 -Wall -Wno-sign-compare -o delly_b200/bin/delly_b200 bindings/delly_b200_main.cpp -I"$HTSINC" \
-    -Ldelly_b200 -l:libdelly_b200.so -Wl,-rpath,'$ORIGIN/..' third_party/_hts/libhts.a -lz -lm -lpthread
+  g++ -std=c++17 -O2 -Wall -Wno-sign-compare -o delly_b200/bin/delly_b200 bindings/delly_b200_main.cpp -I$HTS/include \
+    -Ldelly_b200 -l:libdelly_b200.so -Wl,-rpath,'$ORIGIN/..' $HTS/libhts.a -lz -lm -lpthread
   echo "built delly_b200/bin/delly_b200"
   # synthetic-sample generator for the pipeline benchmarks / whole-file parity tests (tools/simbam.cpp)
-  g++ -std=c++17 -O2 -Wall -o delly_b200/bin/simbam tools/simbam.cpp -I"$HTSINC" third_party/_hts/libhts.a -lz -lm -lpthread
+  g++ -std=c++17 -O2 -Wall -o delly_b200/bin/simbam tools/simbam.cpp -I$HTS/include $HTS/libhts.a -lz -lm -lpthread
   echo "built delly_b200/bin/simbam"
 else
-  echo "htslib headers not present; keeping prebuilt delly_b200/bin/delly_b200 if any"
+  echo "htslib (oracle/_ref/hts) not present; delly_b200/bin/delly_b200 not built" >&2
 fi
